@@ -19,6 +19,8 @@ another BASELINE configuration as the bench line.  Each step uses fresh seeds.
   configs   (default run, 1 GPU) the other four BASELINE configurations, each measured and parity-checked the same way
 
 `--impl reference` times that CPU implementation alone (all host threads) on the same metric/config.
+`--dump-outputs DIR` writes the results of the last timed step as .npy files (see dump_outputs), so that two builds run
+with the same arguments, hence on the same seeds, can be compared output for output.
 Multi-GPU: one process per GPU under torchrun through `ShardedBatchSimulator`: instances sharded with no data-path
 collective; one NCCL all-gather of the per-instance summaries at the end of every step.  "scaling": "weak" (the
 configuration's batch per GPU) unless `--scaling strong` (the configuration's batch split over the GPUs).
@@ -274,6 +276,30 @@ def gpu_arrays(res):
     return {"commit_counts": res.commit_counts, "last_states": res.last_committed_states, "counters": res.counters}
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(res, out_dir, limit_bytes=DUMP_LIMIT_BYTES):
+    """Write what a caller of the timed path receives for one batch (a BatchResult) to out_dir/<name>.npy, all float64:
+    commit_counts [I][N]; last_committed_states_hi and _lo [I][N], the upper and lower 32 bits of the 64-bit state keys (each
+    exact in float64); active_rounds [I]; status [I]; counters [I][12]; and instance [I], the batch index of each row.  When
+    all of it would exceed limit_bytes, the rows are a fixed, seeded sample of the instances, the same one on every run."""
+    states = np.asarray(res.last_committed_states, dtype=np.uint64)
+    arrays = {"commit_counts": res.commit_counts, "last_committed_states_hi": states >> np.uint64(32),
+              "last_committed_states_lo": states & np.uint64(0xFFFFFFFF), "active_rounds": res.active_rounds,
+              "status": res.status, "counters": res.counters}
+    total = len(states)
+    row_bytes = 8 * (1 + sum(int(np.prod(np.shape(a)[1:])) for a in arrays.values()))
+    rows = np.arange(total)
+    if total * row_bytes > limit_bytes:
+        keep = (limit_bytes - 4096) // row_bytes   # 4 KB of headroom for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(total, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "instance.npy"), rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a)[rows].astype(np.float64))
+
+
 def roofline_block(cfg_id, cfg, per_gpu, counters, kernel_ms, kernel_name):
     peak, peak_src = measured_peak_gbs()
     bytes_launch = algorithmic_bytes(counters, cfg["nodes"])
@@ -291,7 +317,7 @@ def roofline_block(cfg_id, cfg, per_gpu, counters, kernel_ms, kernel_name):
     return block
 
 
-def measure_side_config(cfg_id, device, steps=2, warmup=1):
+def measure_side_config(cfg_id, device, steps, warmup):
     """One of the non-headline BASELINE configurations on one GPU: kernel time (CUDA events, seeds resident), e2e time
     (host buffers), full parity and the CPU baseline.  Used for the `configs` block of the default line."""
     import torch
@@ -350,6 +376,7 @@ def emit(line):
 
 
 def main():
+    sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from, which may be read-only
     quiet_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -362,7 +389,13 @@ def main():
                     help="weak: the configuration's batch per GPU; strong: the configuration's batch split over the GPUs")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the oracle (no parity check, no cpu_baseline)")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config block of the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step (rank 0's shard) to "
+                                                          "DIR/<name>.npy as float64, at most 64 MB (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU path; the reference arm times a machine-dependent sample")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -449,6 +482,8 @@ def main():
         flagged += int(((last.status & 0x9E) != 0).sum())  # any LBFT_ST_ERROR_MASK bit (capacity / invariant / epoch)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, args.dump_outputs)
 
     dev_seconds = sum(kernel_ms) / 1e3
     stats = torch.tensor([dev_seconds, e2e_seconds], dtype=torch.float64, device="cuda")
@@ -491,7 +526,7 @@ def main():
                 sim.close()
                 side = {}
                 for k in (1, 2, 4, 5):
-                    side[str(k)] = measure_side_config(k, local_rank)
+                    side[str(k)] = measure_side_config(k, local_rank, args.steps, args.warmup)
                 me = {"workload": cfg["text"], "kernel": kernel, "kernel_ms": k_ms, "value": value, "unit": UNIT,
                       "e2e": line["e2e"]["value"], "events_per_s": line["roofline"]["events_per_s"], "roofline": line["roofline"],
                       "flagged_instances": flagged, "parity": parity, "cpu_baseline": base,

@@ -2,7 +2,7 @@
 
 * ``csrc/liblbft_b200.so`` — the product: sm_100a CUDA kernels + the C ABI of ``include/lbft.h``.
 * ``oracle/liblbft_oracle.so`` and ``tests/hostcore/libhostcore.so`` — test infrastructure only.
-All artefacts are built in-tree (git-ignored, but they travel to the GPU box with the snapshot).
+These three are built in-tree (git-ignored) by ``build()``; nothing that runs later compiles into the tree.
 """
 import os
 import shutil
@@ -77,27 +77,27 @@ def build_oracle(force=False):
     return ORACLE_PATH
 
 
+_NATIVE_ORACLE = {}
+
+
 def build_oracle_native():
-    """The CPU-baseline build of the oracle (-O3 -march=native), compiled on the machine that times it (the GPU box: same
-    image, g++ present) into a host-specific file name so that a copy built for another CPU is never loaded.  Falls back
-    to the portable build if no compiler is available.  Returns (path, flags description)."""
-    import hashlib
-    import platform
-    try:
-        cpu = [ln for ln in open("/proc/cpuinfo") if ln.startswith(("model name", "flags"))][:2]
-    except OSError:
-        cpu = [platform.processor()]
-    tag = hashlib.sha1("".join(cpu).encode()).hexdigest()[:10]
-    path = os.path.join(ORACLE_DIR, "liblbft_oracle_native_%s.so" % tag)
-    srcs = [os.path.join(ORACLE_DIR, f) for f in ("oracle_capi.cpp", "oracle_selftest.cpp", "lbft_oracle.hpp")]
-    if _newer(path, srcs):
-        return path, "-O3 -march=native"
-    try:
-        _run(["make", "-B", "liblbft_oracle_native.so"], ORACLE_DIR)
-        os.replace(os.path.join(ORACLE_DIR, "liblbft_oracle_native.so"), path)
-        return path, "-O3 -march=native"
-    except Exception:
-        return build_oracle(), "-O2 (portable build: native build failed)"
+    """The CPU-baseline build of the oracle (-O3 -march=native), compiled on the machine that times it, once per process.
+    It goes to a fresh private directory from tempfile.mkdtemp (this user's, mode 0700, unpredictable name) that is
+    removed when the process exits: never into the source tree, which bench.py may find read-only, and never a library
+    another user could have placed in a shared location.  Falls back to the portable build if no compiler is available.
+    Returns (path, flags description)."""
+    if "lib" not in _NATIVE_ORACLE:
+        import atexit
+        import tempfile
+        outdir = tempfile.mkdtemp(prefix="lbft_oracle_native_")
+        atexit.register(shutil.rmtree, outdir, True)
+        path = os.path.join(outdir, "liblbft_oracle_native.so")
+        try:
+            _run(["make", "native", "NATIVE_OUT=" + path], ORACLE_DIR)
+            _NATIVE_ORACLE["lib"] = path, "-O3 -march=native"
+        except Exception:
+            _NATIVE_ORACLE["lib"] = build_oracle(), "-O2 (portable build: native build failed)"
+    return _NATIVE_ORACLE["lib"]
 
 
 def build_hostcore(force=False):
