@@ -145,6 +145,38 @@ typedef struct lbft_sim lbft_sim;
  * durations — all libm calls stay on the host), allocate device state.  Does not run anything. */
 int lbft_create(const lbft_config* config, lbft_sim** out_sim);
 
+/* One parameter set of a sweep (lbft_create_sweep): the knobs of a Monte-Carlo study — RandomDelay (simulator.rs:99-106,
+ * or the uniform extension), NodeConfig (node.rs:76-81) and the silent (crashed) nodes — with lbft_config's meaning. */
+typedef struct lbft_param_set {
+  uint32_t struct_size;           /* = sizeof(lbft_param_set); ABI guard                                    */
+  uint32_t delay_kind;            /* LBFT_DELAY_*                                                           */
+  double delay_mean;
+  double delay_variance;
+  int64_t delay_lo, delay_hi;     /* LBFT_DELAY_UNIFORM only                                                */
+  int64_t target_commit_interval;
+  int64_t delta;                  /* > 0                                                                    */
+  double gamma;
+  double lambda;
+  uint64_t silent_mask;           /* bit i set = node i is silent; bits >= num_nodes are refused            */
+} lbft_param_set;
+
+/* Largest num_sets lbft_create_sweep accepts. */
+#define LBFT_MAX_PARAM_SETS 4096u
+
+/* A sweep handle: one batch whose instances run with different parameter sets.  Instance i runs with
+ * sets[set_of_instance[i]] (set_of_instance is a host array of config->num_instances entries, copied): it computes
+ * exactly what instance i of an lbft_create handle computes whose config carries that set's values — same seed stream,
+ * same RNG draws, same results (commit counts, state keys, commit logs, counters, status, active rounds).  The sets
+ * replace config's delay_kind, delay_mean, delay_variance, delay_lo, delay_hi, target_commit_interval, delta, gamma,
+ * lambda and silent: those fields of config are NOT read.  Everything else (num_nodes, max_clock, seeds,
+ * commands_per_epoch, voting_rights, partition plan, capacities, device) is shared by the handle.  Each set is validated
+ * like lbft_create validates a config; LBFT_ERR_INVALID also when config->flags is not 0, when commands_per_epoch <
+ * round_cap (a multi-epoch layout), when num_sets is 0 or above LBFT_MAX_PARAM_SETS, or when a set index is out of
+ * range.  The queue mode and capacities are chosen to fit every set.  Every other entry point works on the handle as
+ * on any other (lbft_set_seeds keeps the set assignment); a sweep handle is never resumable. */
+int lbft_create_sweep(const lbft_config* config, const lbft_param_set* sets, uint32_t num_sets,
+                      const uint32_t* set_of_instance, lbft_sim** out_sim);
+
 /* Simulator::new for every instance followed by loop_until(max_clock) (simulator.rs:200-250,
  * 380-475): copies the seeds host->device, runs the event-loop kernel to completion, copies the
  * per-node summaries (commit counts, last-committed-state keys, counters, status) device->host.

@@ -1,8 +1,8 @@
 """Build recipes for the native pieces (run by ``__graft_entry__.build()``).
 
 * ``csrc/liblbft_b200.so`` — the product: sm_100a CUDA kernels + the C ABI of ``include/lbft.h``.
-* ``oracle/liblbft_oracle.so`` and ``tests/hostcore/libhostcore.so`` — test infrastructure only.
-These three are built in-tree (git-ignored) by ``build()``; nothing that runs later compiles into the tree.
+* ``oracle/liblbft_oracle.so``, ``tests/hostcore/libhostcore.so`` and ``tests/hostcore/libsweepcore.so`` — test infrastructure only.
+These four are built in-tree (git-ignored) by ``build()``; nothing that runs later compiles into the tree.
 """
 import os
 import shutil
@@ -15,11 +15,12 @@ ORACLE_DIR = os.path.join(ROOT, "oracle")
 ORACLE_PATH = os.path.join(ORACLE_DIR, "liblbft_oracle.so")
 HOSTCORE_DIR = os.path.join(ROOT, "tests", "hostcore")
 HOSTCORE_PATH = os.path.join(HOSTCORE_DIR, "libhostcore.so")
+SWEEPCORE_PATH = os.path.join(HOSTCORE_DIR, "libsweepcore.so")
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 # Translation units of the product library: the host runtime (C ABI) and the kernel instantiations, one group per file so
 # that they compile in parallel and the bench kernel (k_fixed.cu) can be rebuilt alone.
-PRODUCT_UNITS = ["lbft_api.cu", "k_fixed.cu", "k_scan.cu", "k_calendar.cu", "k_heap.cu", "k_wide.cu"]
+PRODUCT_UNITS = ["lbft_api.cu", "k_fixed.cu", "k_scan.cu", "k_calendar.cu", "k_heap.cu", "k_wide.cu", "k_sweep.cu", "k_sweep_wide.cu"]
 PRODUCT_HEADERS = ["kernels.cuh", "sim_core.cuh", "sim_params.h", "host_setup.hpp"]
 
 
@@ -112,5 +113,16 @@ def build_hostcore(force=False):
     return HOSTCORE_PATH
 
 
+def build_sweepcore(force=False):
+    """The parameter-sweep state machine for the host (tests/hostcore/sweepcore.cpp), the CPU check of the sweep kernels."""
+    srcs = [os.path.join(HOSTCORE_DIR, "sweepcore.cpp")] + [
+        os.path.join(CSRC, f) for f in ("sim_core.cuh", "sim_params.h", "host_setup.hpp")]
+    if not force and _newer(SWEEPCORE_PATH, srcs):
+        return SWEEPCORE_PATH
+    _run(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-ffp-contract=off", "-Wno-unknown-pragmas", "-DLBFT_CHECK_C1",
+          "-o", SWEEPCORE_PATH, "sweepcore.cpp"], HOSTCORE_DIR)
+    return SWEEPCORE_PATH
+
+
 def build_all(force=False):
-    return build_product(force), build_oracle(force), build_hostcore(force)
+    return build_product(force), build_oracle(force), build_hostcore(force), build_sweepcore(force)

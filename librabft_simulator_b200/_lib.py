@@ -24,6 +24,18 @@ class LbftConfig(ctypes.Structure):
     ]
 
 
+class LbftParamSet(ctypes.Structure):
+    """``lbft_param_set`` of include/lbft.h: one parameter set of a sweep (``lbft_create_sweep``)."""
+    _fields_ = [
+        ("struct_size", c_u32), ("delay_kind", c_u32), ("delay_mean", c_f64), ("delay_variance", c_f64),
+        ("delay_lo", c_i64), ("delay_hi", c_i64), ("target_commit_interval", c_i64), ("delta", c_i64),
+        ("gamma", c_f64), ("lambda_", c_f64), ("silent_mask", c_u64),
+    ]
+
+
+MAX_PARAM_SETS = 4096  # LBFT_MAX_PARAM_SETS
+
+
 class LbftCommit(ctypes.Structure):
     _fields_ = [("proposer", c_u32), ("index", c_u32), ("time", c_i64)]
 
@@ -50,7 +62,7 @@ ST_INVARIANT, ST_EPOCH_CHANGE, ST_DELAY_NEAR_INT, ST_TIME_OVERFLOW = 16, 32, 64,
 ST_ERROR_MASK = ST_ROUND_OVERFLOW | ST_QUEUE_OVERFLOW | ST_PAYLOAD_OVERFLOW | ST_INVARIANT | ST_TIME_OVERFLOW
 
 EXPORTS = [
-    "lbft_create", "lbft_run", "lbft_run_async", "lbft_wait", "lbft_commit_logs", "lbft_upload", "lbft_run_device", "lbft_download", "lbft_commit_counts",
+    "lbft_create", "lbft_create_sweep", "lbft_run", "lbft_run_async", "lbft_wait", "lbft_commit_logs", "lbft_upload", "lbft_run_device", "lbft_download", "lbft_commit_counts",
     "lbft_last_states", "lbft_commit_log", "lbft_round_switches", "lbft_active_rounds", "lbft_counters", "lbft_status", "lbft_timing_info",
     "lbft_memory_info", "lbft_kernel_info", "lbft_run_until", "lbft_snapshot_size", "lbft_snapshot_save", "lbft_snapshot_load", "lbft_set_seeds", "lbft_device_buffer", "lbft_destroy", "lbft_last_error", "lbft_abi_version",
 ]
@@ -76,6 +88,7 @@ def load():
     lib = ctypes.CDLL(LIB_PATH)
     P = ctypes.c_void_p
     lib.lbft_create.argtypes = [ctypes.POINTER(LbftConfig), ctypes.POINTER(P)]
+    lib.lbft_create_sweep.argtypes = [ctypes.POINTER(LbftConfig), ctypes.POINTER(LbftParamSet), c_u32, P, ctypes.POINTER(P)]
     for name in ("lbft_run", "lbft_run_async", "lbft_wait", "lbft_upload", "lbft_run_device", "lbft_download"):
         getattr(lib, name).argtypes = [P]
     for name in ("lbft_commit_counts", "lbft_last_states", "lbft_active_rounds", "lbft_counters", "lbft_status"):

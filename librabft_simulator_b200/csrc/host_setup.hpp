@@ -14,6 +14,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -84,6 +85,19 @@ struct HostSetup {
   bool use_wide = false;      // launch lbft_wide_kernel (one warp per instance) instead of one thread per instance
   bool wide_smem = false;     // ... with the instance state in shared memory (committees of <= 16, short horizons)
   uint32_t wide_group = 32;   // ... lanes per instance: 8 / 16 / 32
+
+  // Parameter sweeps (lbft_create_sweep, build_sweep): the tables of every set, and each instance's set.
+  std::vector<SweepSet> sets;
+  std::vector<uint32_t> set_of;
+  std::vector<double> sweep_thr;
+  std::vector<int32_t> sweep_duration, sweep_period;
+
+  // Events created per simulated ms, the estimate the queue mode is chosen by: ~0.14 N^2 at the reference's 10 ms mean
+  // delay, proportionally more with shorter delays.
+  static double event_rate(const lbft_config& c) {
+    const double mean_delay = c.delay_kind == LBFT_DELAY_UNIFORM ? 0.5 * (double)(c.delay_lo + c.delay_hi) : c.delay_mean;
+    return 0.14 * c.num_nodes * c.num_nodes * (10.0 / (mean_delay < 1.0 ? 1.0 : mean_delay));
+  }
 
   bool build(const lbft_config& c) {
     if (c.struct_size != sizeof(lbft_config)) return fail("lbft_config.struct_size does not match this library (ABI mismatch)");
@@ -204,8 +218,7 @@ struct HostSetup {
     // shortest horizons: 32-bit keys (time:14 | kind:2 | stamp:16) + 16-bit payload words, queue in shared memory
     // (16-bit stamps: ~0.14 N^2 events are created per simulated ms at the reference's 10 ms mean delay, and
     // proportionally more with shorter delays; stay well inside 65 536 — an overflow would be flagged, not silent)
-    const double mean_delay = c.delay_kind == LBFT_DELAY_UNIFORM ? 0.5 * (double)(c.delay_lo + c.delay_hi) : c.delay_mean;
-    const double events_per_ms = 0.14 * N * N * (10.0 / (mean_delay < 1.0 ? 1.0 : mean_delay));
+    const double events_per_ms = event_rate(c);
     if (qscan && c.max_clock < (1 << 14) - 64 && qcap <= 64 && pcap <= 255 && events_per_ms * (double)c.max_clock < 32768.0)
       qscan = 2;
     // the HBM scan queue hands out 22-bit creation stamps: long horizons / very short delays go to the heap or calendar
@@ -278,6 +291,67 @@ struct HostSetup {
     return true;
   }
 
+  // A sweep handle: `c` with the values of set set_of[i] for instance i (its delay fields, target_commit_interval, delta,
+  // gamma, lambda and silent are not read).  Each set is validated and its tables built by build() on the plain
+  // configuration it stands for; the shared part (layout, leader table, weights, kernel family) is built once more for
+  // the set with the highest event rate, with the element-wise largest queue / payload capacities of all the sets:
+  // the queue modes only widen their creation stamps as the event rate grows, so no instance can raise a capacity bit
+  // that its set's plain handle would not raise.
+  bool build_sweep(const lbft_config& c, const lbft_param_set* ps, uint32_t num_sets, const uint32_t* set_index) {
+    if (c.struct_size != sizeof(lbft_config)) return fail("lbft_config.struct_size does not match this library (ABI mismatch)");
+    if (c.flags) return fail("sweep handles are plain one-shot runs: lbft_config.flags must be 0 (no recording, resumable runs or "
+                             "true data-sync)");
+    if (num_sets == 0 || num_sets > LBFT_MAX_PARAM_SETS) return fail("num_sets must be in 1..LBFT_MAX_PARAM_SETS");
+    if (!ps || !set_index) return fail("sets and set_of_instance must not be NULL");
+    for (uint32_t i = 0; i < c.num_instances; i++)
+      if (set_index[i] >= num_sets) {
+        char buf[128];
+        snprintf(buf, sizeof buf, "set_of_instance[%u] = %u is out of range (num_sets = %u)", i, set_index[i], num_sets);
+        return fail(buf);
+      }
+    uint8_t silent[64];
+    uint32_t best = 0, qmax = 0, pmax = 0, qmin = ~0u, pmin = ~0u;
+    double best_rate = -1.0;
+    sets.assign(num_sets, SweepSet{});
+    sweep_thr.clear();
+    sweep_duration.clear();
+    sweep_period.clear();
+    for (uint32_t k = 0; k < num_sets; k++) {
+      char pre[48];
+      snprintf(pre, sizeof pre, "parameter set %u: ", k);
+      if (ps[k].struct_size != sizeof(lbft_param_set)) return fail(std::string(pre) + "struct_size does not match this library (ABI mismatch)");
+      if (c.num_nodes < 64 && (ps[k].silent_mask >> c.num_nodes)) return fail(std::string(pre) + "silent_mask has bits at or above num_nodes");
+      const lbft_config cs = with_set(c, ps[k], silent);
+      HostSetup h;
+      if (!h.build(cs)) return fail(std::string(pre) + h.error);
+      if (h.params.L.epochs > 1)
+        return fail("sweep handles need commands_per_epoch >= round_cap (a single-epoch layout): the sweep kernels have no epoch machinery");
+      const Params& q = h.params;
+      SweepSet& t = sets[k];
+      t.mu = q.mu; t.sigma = q.sigma; t.delay_const_value = q.delay_const_value;
+      t.uni_lo = q.uni_lo; t.uni_span = q.uni_span; t.silent_mask = q.silent_mask;
+      t.delay_kind = q.delay_kind; t.delay_const = q.delay_const; t.delay_kmax = q.delay_kmax; t.tci = q.tci;
+      t.thr_off = (uint32_t)sweep_thr.size();
+      t.tab_off = (uint32_t)sweep_duration.size();
+      sweep_thr.insert(sweep_thr.end(), h.delay_thr.begin(), h.delay_thr.end());
+      sweep_duration.insert(sweep_duration.end(), h.duration.begin(), h.duration.end());
+      sweep_period.insert(sweep_period.end(), h.period.begin(), h.period.end());
+      const double rate = event_rate(cs);
+      if (rate > best_rate) { best_rate = rate; best = k; }
+      qmax = std::max(qmax, q.L.queue_cap); qmin = std::min(qmin, q.L.queue_cap);
+      pmax = std::max(pmax, q.L.payload_cap); pmin = std::min(pmin, q.L.payload_cap);
+    }
+    lbft_config cb = with_set(c, ps[best], silent);
+    if (qmin != qmax) cb.queue_cap = qmax;
+    if (pmin != pmax) cb.payload_cap = pmax;
+    if (!build(cb)) return false;
+    if (params.L.queue_cap < qmax || params.L.payload_cap < pmax) return fail("sweep capacities below a set's own (internal error)");
+    // Sparse thread-kernel tiles have no sweep instantiation: those shapes run the lane-group kernel.
+    if (!use_wide && tile_stride != 32) { use_wide = true; tile_stride = 1; }
+    set_of.assign(set_index, set_index + c.num_instances);
+    return true;
+  }
+
   // LogNormal delay without a device-side exp(): the reference truncates exp(mu + sigma*z) to an integer
   // (simulator.rs:115-117), so only the integer part matters.  delay_thr[k] is the smallest double z with
   // (exp(mu + sigma*z) as i64) >= k, found by bisection over the doubles with the HOST libm — the very
@@ -342,9 +416,24 @@ struct HostSetup {
   }
 
  private:
-  bool fail(const char* msg) {
+  bool fail(const std::string& msg) {
     error = msg;
     return false;
+  }
+  // The plain configuration a parameter set stands for (`silent` receives the set's mask as lbft_config.silent).
+  static lbft_config with_set(lbft_config c, const lbft_param_set& s, uint8_t (&silent)[64]) {
+    c.delay_kind = s.delay_kind;
+    c.delay_mean = s.delay_mean;
+    c.delay_variance = s.delay_variance;
+    c.delay_lo = s.delay_lo;
+    c.delay_hi = s.delay_hi;
+    c.target_commit_interval = s.target_commit_interval;
+    c.delta = s.delta;
+    c.gamma = s.gamma;
+    c.lambda = s.lambda;
+    for (uint32_t i = 0; i < 64; i++) silent[i] = (uint8_t)((s.silent_mask >> i) & 1u);
+    c.silent = s.silent_mask ? silent : nullptr;
+    return c;
   }
 };
 

@@ -5,7 +5,8 @@
 //
 // Both do init -> event loop -> read-out in a single launch.  The instantiations are spread over several .cu files
 // (k_fixed.cu, k_scan.cu, k_calendar.cu, k_heap.cu, k_wide.cu) so that they compile in parallel and the bench kernel
-// can be rebuilt alone; lbft_api.cu only sees the launch_* functions declared at the end.
+// can be rebuilt alone; lbft_api.cu only sees the launch_* functions declared at the end.  The kernels of parameter
+// sweeps (Core SW = true) are defined in k_sweep.cu / k_sweep_wide.cu.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -161,6 +162,7 @@ struct KernelSel {
   int qmode;   // Layout::queue_scan
   int fixed;   // FX_* (sim_params.h): the instantiation with that compile-time layout; FX_NONE = generic
   bool rec, res;
+  bool sweep;  // parameter sweep (lbft_create_sweep): lbft_sweep_kernel / lbft_sweep_wide_kernel (k_sweep*.cu)
 };
 
 // One per translation unit; each returns cudaErrorInvalidValue if the selection is not one of its instantiations.
@@ -169,6 +171,8 @@ cudaError_t launch_scan(const KernelSel& k, const Params& P, cudaStream_t stream
 cudaError_t launch_calendar(const KernelSel& k, const Params& P, cudaStream_t stream);
 cudaError_t launch_heap(const KernelSel& k, const Params& P, cudaStream_t stream);
 cudaError_t launch_wide(const KernelSel& k, const Params& P, cudaStream_t stream);
+cudaError_t launch_sweep(const KernelSel& k, const Params& P, cudaStream_t stream);
+cudaError_t launch_sweep_wide(const KernelSel& k, const Params& P, cudaStream_t stream);
 
 // Shared by the launchers of the thread-per-instance kernel.
 template <int NMAX, int QM, int TILE, int FX = FX_NONE>

@@ -74,6 +74,12 @@ struct lbft_sim {
   int32_t* d_period = nullptr;
   uint32_t* d_weights = nullptr;
   double* d_delay_thr = nullptr;
+  // sweep handles (lbft_create_sweep): the per-set tables and each instance's set
+  SweepSet* d_sets = nullptr;
+  uint32_t* d_set_of = nullptr;
+  double* d_sweep_thr = nullptr;
+  int32_t* d_sweep_duration = nullptr;
+  int32_t* d_sweep_period = nullptr;
   uint32_t* d_state = nullptr;
   uint32_t* d_commit_counts = nullptr;
   uint32_t* d_lc_round = nullptr;
@@ -120,6 +126,7 @@ static void free_all(lbft_sim* s) {
   cudaFree(s->d_period); cudaFree(s->d_weights); cudaFree(s->d_delay_thr); cudaFree(s->d_state); cudaFree(s->d_summary);
   cudaFree(s->d_lc_round); cudaFree(s->d_counters); cudaFree(s->d_status);
   cudaFree(s->d_error); cudaFree(s->d_logs);
+  cudaFree(s->d_sets); cudaFree(s->d_set_of); cudaFree(s->d_sweep_thr); cudaFree(s->d_sweep_duration); cudaFree(s->d_sweep_period);
   for (int b = 0; b < 2; b++) {
     cudaFreeHost(s->h_seeds[b]);
     HostResults& r = s->res[b];
@@ -205,6 +212,8 @@ static int need_idle(lbft_sim* s) {
   return LBFT_OK;
 }
 
+static int create_handle(lbft_sim* s, const lbft_config* config, lbft_sim** out_sim);
+
 extern "C" {
 
 uint32_t lbft_abi_version(void) { return LBFT_ABI_VERSION; }
@@ -225,6 +234,27 @@ int lbft_create(const lbft_config* config, lbft_sim** out_sim) {
     return set_error(LBFT_ERR_INVALID, "recording / resumable handles need commands_per_epoch >= round_cap: the kernels with the epoch "
                                        "machinery (node.rs:329-348) are built for plain runs only");
   }
+  return create_handle(s, config, out_sim);
+}
+
+int lbft_create_sweep(const lbft_config* config, const lbft_param_set* sets, uint32_t num_sets, const uint32_t* set_of_instance,
+                      lbft_sim** out_sim) {
+  if (!config || !out_sim) return set_error(LBFT_ERR_INVALID, "config and out_sim must not be NULL");
+  *out_sim = nullptr;
+  lbft_sim* s = new (std::nothrow) lbft_sim();
+  if (!s) return set_error(LBFT_ERR_NOMEM, "out of host memory");
+  if (!s->hs.build_sweep(*config, sets, num_sets, set_of_instance)) {
+    std::string e = s->hs.error;
+    delete s;
+    return set_error(LBFT_ERR_INVALID, e);
+  }
+  return create_handle(s, config, out_sim);
+}
+
+}  // extern "C"
+
+// The device side of lbft_create / lbft_create_sweep once the host setup has been built and validated.
+static int create_handle(lbft_sim* s, const lbft_config* config, lbft_sim** out_sim) {
   s->I = config->num_instances;
   s->N = config->num_nodes;
   s->device = config->device;
@@ -293,6 +323,20 @@ int lbft_create(const lbft_config* config, lbft_sim** out_sim) {
   CREATE_TRY(cudaMemcpy(s->d_weights, s->hs.weights.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice));
   if (s->d_delay_thr)
     CREATE_TRY(cudaMemcpy(s->d_delay_thr, s->hs.delay_thr.data(), s->hs.delay_thr.size() * sizeof(double), cudaMemcpyHostToDevice));
+  const HostSetup& hs = s->hs;
+  if (!hs.sets.empty()) {
+    CREATE_TRY(dev_alloc(s, &s->d_sets, hs.sets.size()));
+    CREATE_TRY(dev_alloc(s, &s->d_set_of, I));
+    CREATE_TRY(dev_alloc(s, &s->d_sweep_duration, hs.sweep_duration.size()));
+    CREATE_TRY(dev_alloc(s, &s->d_sweep_period, hs.sweep_period.size()));
+    if (!hs.sweep_thr.empty()) CREATE_TRY(dev_alloc(s, &s->d_sweep_thr, hs.sweep_thr.size()));
+    CREATE_TRY(cudaMemcpy(s->d_sets, hs.sets.data(), hs.sets.size() * sizeof(SweepSet), cudaMemcpyHostToDevice));
+    CREATE_TRY(cudaMemcpy(s->d_set_of, hs.set_of.data(), I * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    CREATE_TRY(cudaMemcpy(s->d_sweep_duration, hs.sweep_duration.data(), hs.sweep_duration.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    CREATE_TRY(cudaMemcpy(s->d_sweep_period, hs.sweep_period.data(), hs.sweep_period.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    if (s->d_sweep_thr)
+      CREATE_TRY(cudaMemcpy(s->d_sweep_thr, hs.sweep_thr.data(), hs.sweep_thr.size() * sizeof(double), cudaMemcpyHostToDevice));
+  }
 #undef CREATE_TRY
   s->P = s->hs.params;
   s->P.seeds = s->d_seeds;
@@ -311,9 +355,17 @@ int lbft_create(const lbft_config* config, lbft_sim** out_sim) {
   s->P.out_status = s->d_status;
   s->P.out_rounds = s->d_rounds;
   s->P.out_error = s->d_error;
+  s->P.sweep_sets = s->d_sets;
+  s->P.set_of = s->d_set_of;
+  s->P.sweep_thr = s->d_sweep_thr;
+  s->P.sweep_duration = s->d_sweep_duration;
+  s->P.sweep_period = s->d_sweep_period;
+  s->P.num_sets = (uint32_t)hs.sets.size();
   *out_sim = s;
   return LBFT_OK;
 }
+
+extern "C" {
 
 int lbft_set_seeds(lbft_sim* s, const uint64_t* seeds) {
   if (!s || !seeds) return set_error(LBFT_ERR_INVALID, "NULL argument");
@@ -431,6 +483,7 @@ static KernelSel select_kernel(const lbft_sim* s) {
   k.nmax = (k.qmode == 1 || k.qmode == 2) ? 16 : (s->N <= 16 ? 16 : (s->N <= 32 ? 32 : 64));
   k.rec = s->P.record_rs != 0;
   k.res = s->P.resumable != 0;
+  k.sweep = s->P.num_sets != 0;
   // shapes with a kernel instantiation with compile-time field offsets (sim_params.h fixed_layout): the handle's layout must
   // be bit-identical and the delay model the reference's (LogNormal served by the threshold table)
   constexpr Layout kDefault4 = fixed_layout(FX_DEFAULT4), kPart7 = fixed_layout(FX_PART7), kCommittee64 = fixed_layout(FX_COMMITTEE64);
@@ -438,6 +491,7 @@ static KernelSel select_kernel(const lbft_sim* s) {
   const bool plain_model = table_delay && s->P.delay_kmax + 2 <= kThrSmem && s->P.silent_mask == 0;
   const bool plain_handle = !k.rec && !k.res && !k.tds && !k.epochs;
   k.fixed = FX_NONE;
+  if (k.sweep) return k;  // (the sweep kernels have no compile-time layouts)
   if (!k.wide && k.qmode == 2 && plain_model && plain_handle && memcmp(&s->P.L, &kDefault4, sizeof(Layout)) == 0) k.fixed = FX_DEFAULT4;
   else if (!k.wide && k.qmode == 3 && k.tile == 8 && plain_model && plain_handle && memcmp(&s->P.L, &kPart7, sizeof(Layout)) == 0) k.fixed = FX_PART7;
   else if (k.wide && k.qmode == 3 && k.group == 8 && !k.smem && table_delay && plain_handle && memcmp(&s->P.L, &kCommittee64, sizeof(Layout)) == 0)
@@ -450,7 +504,11 @@ static KernelSel select_kernel(const lbft_sim* s) {
 static std::string kernel_name(const lbft_sim* s) {
   const KernelSel k = select_kernel(s);
   char buf[96];
-  if (k.wide)
+  if (k.sweep && k.wide)
+    snprintf(buf, sizeof buf, "lbft_sweep_wide_kernel<%d,%d,%s,%d>", k.nmax, k.qmode, k.smem ? "true" : "false", k.group);
+  else if (k.sweep)
+    snprintf(buf, sizeof buf, "lbft_sweep_kernel<%d,%d>", k.nmax, k.qmode);
+  else if (k.wide)
     snprintf(buf, sizeof buf, "lbft_wide_kernel<%d,%d,%s,%d,%s,%d>", k.nmax, k.qmode, k.smem ? "true" : "false", k.group, k.epochs ? "true" : "false", k.fixed);
   else
     snprintf(buf, sizeof buf, "lbft_event_loop_kernel<%d,%d,%d,%s,%s,%s,%s,%d>", k.nmax, k.qmode, k.fixed, k.rec ? "true" : "false",
@@ -464,7 +522,8 @@ static int enqueue_kernel(lbft_sim* s) {
   CUDA_TRY(cudaMemsetAsync(s->d_error, 0, sizeof(uint32_t), s->stream));
   CUDA_TRY(cudaEventRecord(s->ev[2], s->stream));
   const KernelSel k = select_kernel(s);
-  cudaError_t e = k.wide ? launch_wide(k, s->P, s->stream)
+  cudaError_t e = k.sweep ? (k.wide ? launch_sweep_wide(k, s->P, s->stream) : launch_sweep(k, s->P, s->stream))
+                  : k.wide ? launch_wide(k, s->P, s->stream)
                   : k.fixed == FX_DEFAULT4 ? launch_fixed(k, s->P, s->stream)
                   : (k.qmode == 1 || k.qmode == 2) ? launch_scan(k, s->P, s->stream)
                   : k.qmode == 3 ? launch_calendar(k, s->P, s->stream)

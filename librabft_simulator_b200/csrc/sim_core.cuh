@@ -340,10 +340,13 @@ LBFT_COLD PartitionSpan partition_span(Mem m, uint32_t part_base, uint32_t windo
 // HBM block: the first hop of every pop and the occupancy test of every push become shared-memory accesses, and a push
 // into an empty list issues no load at all.  Sparse-tile thread kernels and the wide kernels (a handful of instances per
 // warp: (max_clock + 8) / 8 words each fit); plain one-shot runs only (nothing is kept between launches).
+// SW: parameter sweep (lbft_create_sweep) — the delay model, NodeConfig (tci, duration / period tables) and silent set come
+// from the instance's SweepSet (select_set, before init) instead of the launch's Params.  With SW = false nothing changes.
 template <class Mem, int NMAX, int QMODE, int FX = 0, bool REC = false, bool RES = false, int G = 1, bool EP = false,
-          bool TDS = false, bool KS = false>
+          bool TDS = false, bool KS = false, bool SW = false>
 struct Core {
   static_assert(!KS || (QMODE == 3 && !RES), "shared-memory occupancy words: calendar queue, one-shot runs");
+  static_assert(!(SW && (FX != FX_NONE || REC || RES || EP || TDS)), "sweeps: plain single-epoch generic kernels only");
   static constexpr bool FIXED = FX != FX_NONE;                               // compile-time layout, reference delay model
   static constexpr bool MAY_SILENT = FX == FX_NONE || FX == FX_COMMITTEE64;  // silent nodes (extension D.2) reachable
   static_assert(!(FIXED && EP), "the compile-time layout is single-epoch");
@@ -402,6 +405,39 @@ struct Core {
       : P(p), L(FIXED ? fixed_layout(FX) : p.L), m(mem), zx(zx_), zf(zf_), thr(thr_), sk(sk_), sd(sd_) {}
 
   // ------------------------------------------------------------------------------------------
+  // the per-set values (SW) or the launch's (otherwise)
+  // ------------------------------------------------------------------------------------------
+  const SweepSet* ss = nullptr;  // SW: this instance's parameter set (read through L1; only the pointer stays in registers)
+  LBFT_HD void select_set(uint32_t set) {
+    ss = P.sweep_sets + set;
+    thr = P.sweep_thr + ss->thr_off;
+  }
+#define LBFT_SET_VALUE(T, f) \
+  LBFT_HD T f() const {      \
+    if constexpr (SW) return ss->f; \
+    else return P.f;         \
+  }
+  LBFT_SET_VALUE(uint32_t, delay_kind)
+  LBFT_SET_VALUE(uint32_t, delay_const)
+  LBFT_SET_VALUE(int64_t, delay_const_value)
+  LBFT_SET_VALUE(uint32_t, delay_kmax)
+  LBFT_SET_VALUE(double, mu)
+  LBFT_SET_VALUE(double, sigma)
+  LBFT_SET_VALUE(uint64_t, uni_lo)
+  LBFT_SET_VALUE(uint64_t, uni_span)
+  LBFT_SET_VALUE(int32_t, tci)
+  LBFT_SET_VALUE(uint64_t, silent_mask)
+#undef LBFT_SET_VALUE
+  LBFT_HD int32_t round_duration(uint32_t n) const {
+    if constexpr (SW) return P.sweep_duration[ss->tab_off + n];
+    else return P.duration[n];
+  }
+  LBFT_HD int32_t round_period(uint32_t n) const {
+    if constexpr (SW) return P.sweep_period[ss->tab_off + n];
+    else return P.period[n];
+  }
+
+  // ------------------------------------------------------------------------------------------
   // RNG (rand_xoshiro 0.6.0 / rand 0.8.3 / rand_distr 0.4.0)
   // ------------------------------------------------------------------------------------------
   LBFT_HD void seed_rng(uint64_t seed, uint64_t& a, uint64_t& b, uint64_t& c, uint64_t& d) const {
@@ -453,8 +489,8 @@ struct Core {
   // (exp(mu + sigma*z) as i64) == number of thresholds <= z; the thresholds were bisected on the host
   // with the host libm, so this is exact.  Any starting guess works; the walk fixes it up.
   LBFT_HD int32_t delay_from_z(double z) const {
-    float g = expf((float)P.mu + (float)P.sigma * (float)z);
-    int32_t k = g < (float)P.delay_kmax ? (int32_t)g : (int32_t)P.delay_kmax;
+    float g = expf((float)mu() + (float)sigma() * (float)z);
+    int32_t k = g < (float)delay_kmax() ? (int32_t)g : (int32_t)delay_kmax();
     if (k < 0) k = 0;
     while (z >= thr[k + 1]) k++;
     while (z < thr[k]) k--;
@@ -462,11 +498,11 @@ struct Core {
   }
   // GlobalTime::add_delay (simulator.rs:110-118): returns the delay in ms.
   LBFT_HD int32_t sample_delay() {
-    if (!FIXED && P.delay_kind == 1u) return (int32_t)(P.uni_lo + gen_range_u64(P.uni_span));
+    if (!FIXED && delay_kind() == 1u) return (int32_t)(uni_lo() + gen_range_u64(uni_span()));
     double z = standard_normal();
-    if (!FIXED && P.delay_const) return (int32_t)P.delay_const_value;  // sigma == 0: exp(mu) evaluated by the host libm
-    if (FIXED || P.delay_kmax) return delay_from_z(z);
-    int64_t r = delay_via_exp(P.mu, P.sigma, z);
+    if (!FIXED && delay_const()) return (int32_t)delay_const_value();  // sigma == 0: exp(mu) evaluated by the host libm
+    if (FIXED || delay_kmax()) return delay_from_z(z);
+    int64_t r = delay_via_exp(mu(), sigma(), z);
     if (r & (1LL << 62)) status |= ST_DELAY_NEAR_INT;
     if (r & (1LL << 61)) status |= ST_TIME_OVERFLOW;
     return (int32_t)(r & 0x7fffffff);
@@ -1066,8 +1102,8 @@ struct Core {
       d.f[F_FLAGS] = (d.f[F_FLAGS] & ~(0xffu << FL_LEADER_SHIFT)) | (ld << FL_LEADER_SHIFT);
       uint32_t base = d.f[F_HCR] > 0 ? d.f[F_HCR] + 2 : 0;  // duration(), :111-124
       if (!(active > base)) { status |= ST_INVARIANT; base = active - 1; }
-      d.f[F_PM_DUR] = (uint32_t)P.duration[active - base];
-      d.f[F_PM_PERIOD] = (uint32_t)P.period[active - base];
+      d.f[F_PM_DUR] = (uint32_t)round_duration(active - base);
+      d.f[F_PM_PERIOD] = (uint32_t)round_period(active - base);
       if (ld != n) a.send_to = (int32_t)ld;
     }
     const uint32_t leader = leader_of(d);
@@ -1144,10 +1180,10 @@ struct Core {
       d.f[F_TRK_TIME] = (uint32_t)clk;
     }
     int32_t tl = (int32_t)d.f[F_TRK_TIME] > (int32_t)d.f[F_LQA] ? (int32_t)d.f[F_TRK_TIME] : (int32_t)d.f[F_LQA];
-    int32_t deadline = tl + P.tci;
+    int32_t deadline = tl + tci();
     if (clk >= deadline) {
       a.query_all = true;
-      deadline = clk + P.tci;
+      deadline = clk + tci();
     }
     if (deadline < a.next) a.next = deadline;
     if (a.query_all) d.f[F_LQA] = (uint32_t)clk;
@@ -1353,8 +1389,8 @@ struct Core {
     // event up to max_clock is popped before a one-shot run ends — and keep the event, a third of the 64-author
     // configuration's traffic, out of the queue and out of the snapshot's reference count.  It still takes its creation
     // stamp and its delay draw.  Not while recording / resumable / true-data-sync (every pop is observable there).
-    if (LBFT_ELIDE_SILENT && ELIDE && !TDS && MAY_SILENT && P.silent_mask && kind != EV_RESPONSE &&
-        ((P.silent_mask >> (kind == EV_NOTIFY ? receiver : sender)) & 1)) {
+    if (LBFT_ELIDE_SILENT && ELIDE && !TDS && MAY_SILENT && silent_mask() && kind != EV_RESPONSE &&
+        ((silent_mask() >> (kind == EV_NOTIFY ? receiver : sender)) & 1)) {
       stamp++;
       if (stamp >= kStampLimit) status |= ST_QUEUE_OVERFLOW;
       if (t <= P.max_clock) {
@@ -1481,9 +1517,9 @@ struct Core {
       proc2 += kind == EV_RESPONSE;
       proc3 += kind == EV_TIMER;
       // EXTENSION D.2: silent nodes handle nothing and answer no request
-      if (MAY_SILENT && P.silent_mask) {
-        bool drop = (P.silent_mask >> receiver) & 1;
-        if (kind == EV_REQUEST && ((P.silent_mask >> sender) & 1)) drop = true;
+      if (MAY_SILENT && silent_mask()) {
+        bool drop = (silent_mask() >> receiver) & 1;
+        if (kind == EV_REQUEST && ((silent_mask() >> sender) & 1)) drop = true;
         if (drop) {
           if (kind == EV_NOTIFY || (TDS && slot != PAY_NONE)) pay_unref(slot, m.ld(L.pay_base + slot * L.pay_words + 2));
           continue;
@@ -1577,7 +1613,7 @@ struct Core {
         // Wide kernel, table-served LogNormal delay: the normal deviates of the fan-out are drawn first (the RNG stream is
         // sequential), then each lane turns its share of them into delays, then the events are queued in list order.
         // Nothing else draws from the stream or takes a creation stamp in between, so the order of both is unchanged.
-        const bool staged = WIDE && list.len > 1 && (FIXED || (P.delay_kind == 0u && !P.delay_const && P.delay_kmax != 0));
+        const bool staged = WIDE && list.len > 1 && (FIXED || (delay_kind() == 0u && !delay_const() && delay_kmax() != 0));
         if (staged) {
           for (uint32_t i = 0; i < list.len; i++) ws->z[i] = standard_normal();
           grp_sync();

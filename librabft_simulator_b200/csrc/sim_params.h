@@ -185,6 +185,19 @@ LBFT_LAYOUT_FN uint32_t res_area_base(const Layout& L, bool record_rs) {
   return rs_table_base(L) + (record_rs ? L.num_nodes * (L.round_cap + 1) : 0);
 }
 
+// One parameter set of a sweep handle (lbft_create_sweep): the values of Params below that a set replaces for the
+// instances assigned to it, as HostSetup::build computed them from the set's own lbft_config.
+struct SweepSet {
+  double mu, sigma;
+  int64_t delay_const_value;
+  uint64_t uni_lo, uni_span;
+  uint64_t silent_mask;
+  uint32_t delay_kind, delay_const, delay_kmax;
+  int32_t tci;
+  uint32_t thr_off;  // first element of this set's delay thresholds in Params::sweep_thr (delay_kmax > 0)
+  uint32_t tab_off;  // first element of this set's round_cap + 1 row in Params::sweep_duration / sweep_period
+};
+
 // Everything the kernel needs that is uniform over the launch.
 struct Params {
   Layout L;
@@ -233,6 +246,16 @@ struct Params {
   uint32_t* out_rounds;  // [I] max over nodes of the pacemaker's active round = counters[6] (the unit of the throughput metric)
   uint32_t* out_error;   // [1] OR of the status words of every instance that ended with an error bit: the host looks at one
                          //     word instead of scanning I statuses
+  // parameter sweeps (appended: nothing above moves); null / 0 on plain handles.  Only the sweep kernels read them: the
+  // instance's set replaces delay_kind .. delay_const_value, mu, sigma, uni_lo, uni_span, tci, silent_mask, delay_kmax,
+  // delay_thr, duration and period above.
+  const SweepSet* sweep_sets;    // [num_sets]
+  const uint32_t* set_of;        // [num_instances] index of each instance's set
+  const double* sweep_thr;       // the sets' delay threshold tables, back to back (SweepSet::thr_off)
+  const int32_t* sweep_duration; // [num_sets][round_cap + 1]
+  const int32_t* sweep_period;   // [num_sets][round_cap + 1]
+  uint32_t num_sets;
+  uint32_t pad3;
 };
 
 }  // namespace lbft

@@ -53,6 +53,24 @@ class NodeConfig:
 
 
 @dataclass(frozen=True)
+class ParamSet:
+    """One parameter set of a sweep: the knobs a Monte-Carlo study moves (network delay, pacemaker ``NodeConfig``, silent
+    nodes).  ``silent`` is ``None`` or a per-node sequence of flags, like ``BatchSimulator(silent=...)``."""
+    network_delay: RandomDelay = RandomDelay()
+    node_config: NodeConfig = NodeConfig()
+    silent: tuple = None
+
+    def to_c(self):
+        s = _lib.LbftParamSet()
+        s.struct_size = ctypes.sizeof(_lib.LbftParamSet)
+        d, n = self.network_delay, self.node_config
+        s.delay_kind, s.delay_mean, s.delay_variance, s.delay_lo, s.delay_hi = d.kind, d.mean, d.variance, d.lo, d.hi
+        s.target_commit_interval, s.delta, s.gamma, s.lambda_ = n.target_commit_interval, n.delta, n.gamma, n.lambda_
+        s.silent_mask = 0 if self.silent is None else sum(1 << i for i, f in enumerate(self.silent) if f)
+        return s
+
+
+@dataclass(frozen=True)
 class GlobalTime:
     """``GlobalTime(i64)`` (simulator.rs:35-37)."""
     value: int
@@ -105,6 +123,8 @@ class BatchResult:
         #: max over nodes of ``ActiveRound::active_round()`` per instance (simulator.rs:86-88)
         self.active_rounds = sim._fetch("lbft_active_rounds", np.uint32, (I,))
         self.status = sim._fetch("lbft_status", np.uint32, (I,))
+        #: parameter set of each instance (sweeps; ``None`` for a plain batch)
+        self.set_index = None if sim.set_index is None else sim.set_index.copy()
         self._counters = None
 
     @property
@@ -141,12 +161,17 @@ class BatchResult:
 
 
 class BatchSimulator:
-    """Many independent ``Simulator`` instances (one per seed) on one GPU."""
+    """Many independent ``Simulator`` instances (one per seed) on one GPU.
+
+    ``param_sets`` (a sequence of ``ParamSet``) makes the batch a parameter sweep: instance i runs with
+    ``param_sets[set_index[i]]`` instead of ``network_delay`` / ``node_config`` / ``silent`` (which must then keep their
+    defaults) and computes exactly what a plain batch with that set would compute for its seed.  ``set_index`` defaults to
+    ``arange(num_instances) % len(param_sets)``."""
 
     def __init__(self, seeds, num_nodes, network_delay=RandomDelay(), node_config=NodeConfig(),
                  commands_per_epoch=30000, voting_rights=None, silent=None, partition_windows=0,
                  partition_max_len=0, device=0, round_cap=0, queue_cap=0, payload_cap=0, record_round_switches=False, resumable=False,
-                 true_data_sync=False):
+                 true_data_sync=False, param_sets=None, set_index=None):
         self._lib = _lib.load()
         self.record_round_switches = bool(record_round_switches)  # LBFT_FLAG_ROUND_SWITCHES (DataWriter, data_writer.rs)
         self.resumable = bool(resumable)  # LBFT_FLAG_RESUMABLE: run_until / snapshot / restore
@@ -162,6 +187,19 @@ class BatchSimulator:
         self.silent = None if silent is None else np.ascontiguousarray(silent, dtype=np.uint8)
         self.partition_windows, self.partition_max_len = int(partition_windows), int(partition_max_len)
         self.device, self.round_cap, self.queue_cap, self.payload_cap = int(device), int(round_cap), int(queue_cap), int(payload_cap)
+        self.param_sets, self.set_index = None, None
+        if param_sets is not None:
+            if network_delay != RandomDelay() or node_config != NodeConfig() or silent is not None:
+                raise ValueError("network_delay, node_config and silent come from param_sets in a sweep: leave them at their defaults")
+            self.param_sets = list(param_sets)
+            if not self.param_sets or any(not isinstance(p, ParamSet) for p in self.param_sets):
+                raise ValueError("param_sets must be a non-empty sequence of ParamSet")
+            idx = np.arange(self.num_instances) % len(self.param_sets) if set_index is None else set_index
+            self.set_index = np.ascontiguousarray(np.asarray(idx).reshape(-1), dtype=np.uint32)
+            if self.set_index.shape[0] != self.num_instances:
+                raise ValueError("set_index needs one entry per seed (%d)" % self.num_instances)
+        elif set_index is not None:
+            raise ValueError("set_index needs param_sets")
         self._handle = None
         self._generation = 0   # bumped by every run: results of an older run know they are stale
         self.timing = None
@@ -192,7 +230,12 @@ class BatchSimulator:
         self.close()
         handle = ctypes.c_void_p()
         cfg = self.make_config(max_clock)
-        _lib.check(self._lib.lbft_create(ctypes.byref(cfg), ctypes.byref(handle)))
+        if self.param_sets is None:
+            _lib.check(self._lib.lbft_create(ctypes.byref(cfg), ctypes.byref(handle)))
+        else:
+            sets = (_lib.LbftParamSet * len(self.param_sets))(*[p.to_c() for p in self.param_sets])
+            _lib.check(self._lib.lbft_create_sweep(ctypes.byref(cfg), sets, len(self.param_sets),
+                                                   ctypes.c_void_p(self.set_index.ctypes.data), ctypes.byref(handle)))
         self._handle = handle
         return self
 

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Compare the SASS of every lbft_event_loop_kernel instantiation in two builds of the library (addresses and
-encodings stripped).  Usage: python tools/sass_compare.py OLD.so NEW.so"""
+"""Compare the SASS of every kernel two builds of the library have in common (matched by mangled symbol name; addresses
+and encodings stripped).  Usage: python tools/sass_compare.py OLD.so NEW.so"""
 import re
 import subprocess
 import sys
@@ -22,16 +22,12 @@ def kernels(path):
     return res
 
 
-def key(name):  # <NMAX, QMODE, FIXED, REC, RES>; REC / RES default to 0 for builds that predate them
-    m = re.search(r"kernelILi(\d+)ELi(\d)ELb([01])E(?:Lb([01])E)?(?:Lb([01])E)?", name)
-    return None if not m else (int(m.group(1)), int(m.group(2)), int(m.group(3)), int(m.group(4) or 0), int(m.group(5) or 0))
-
-
-old = {key(k): v for k, v in kernels(sys.argv[1]).items() if key(k)}
-new = {key(k): v for k, v in kernels(sys.argv[2]).items() if key(k)}
-for k in sorted(new):
+old, new = kernels(sys.argv[1]), kernels(sys.argv[2])
+for k in sorted(set(old) | set(new)):
     if k not in old:
-        verdict = "new instantiation"
+        verdict = "new"
+    elif k not in new:
+        verdict = "removed"
     else:
         verdict = "IDENTICAL" if old[k] == new[k] else "differs (%d -> %d instructions)" % (len(old[k]), len(new[k]))
-    print("<%d,%d,%d,%d,%d> %6d instructions  %s" % (k + (len(new[k]), verdict)))
+    print("%-90s %6d instructions  %s" % (k, len(new.get(k, old.get(k))), verdict))
